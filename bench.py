@@ -69,7 +69,12 @@ def parse_args():
     ap.add_argument("--mp3-frames", type=int, default=6)
     ap.add_argument("--am-streams", type=int, default=256)
     ap.add_argument("--am-frames", type=int, default=12)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the records of the last timed step as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def make_captures(distinct: int, frames: int, base_seed: int = 1234):
@@ -151,7 +156,7 @@ def l2_leg(args):
     pk = [ev for r in l2 for t, ev in r["events"] if t == eng.EV_PACKET]
     assert len(l2) >= 2 and len(pk) >= 30 * (len(l2) - 1), (len(l2), len(pk))
     assert all(p["flags"] == 0 for p in pk) and not any(r["flags"] for r in l2)
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     ms_off = timed(False, steps)
     ms_on = timed(True, steps)
     e.set_profiling(True)
@@ -208,7 +213,7 @@ def mp3_leg(args):
           for rr in recs]
     assert nf[0][0] >= F - 1 and nf[0][1] >= 8 * (F - 2) - 2, nf[0]         # P3 output starts after two frames of interleaver fill
     first = [record_digest(r) for r in recs]
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     tot = sum(step()[0] for _ in range(steps))
     res = 0.0
     for _ in range(steps):
@@ -263,7 +268,7 @@ def am_leg(args, engine_factory=None):
     assert len(p1) >= 8 * (F - 8), f"{len(p1)} AM P1 frames decoded from {F} transmitted L1 frames"
     gate = parity_gate(views, recs, am=True, what="am_config4")   # every channel: P1 / P3 / PIDS PDUs in order == oracle
     first = [record_digest(r) for r in recs]
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     tot = proc = 0.0
     for _ in range(steps):
         a, b, _ = step()
@@ -407,7 +412,7 @@ def chan_leg(args):
         for _ in range(3):
             run()
         torch.cuda.synchronize()
-        steps = max(5, min(args.steps, 20))
+        steps = args.steps
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record(stream)
         for _ in range(steps):
@@ -510,6 +515,72 @@ def parity_gate(views, recs_per_stream, am=False, what=""):
                                  f"engine {got[k:k + 2]} ({len(got)} records) vs oracle {w[k:k + 2]} ({len(w)})")
         npdu += sum(1 for g in got if g[0] in "FP")
     return {"ok": True, "streams_checked": len(views), "distinct_views": ndistinct, "pdus_compared": npdu, "oracle": kind}
+
+
+DUMP_BUDGET_BYTES = 63 * 10**6           # leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(out_dir, recs_per_stream):
+    """Writes what a caller of the timed path receives - every stream's parsed records after the last timed step -
+    as float arrays under out_dir, one row per record, streams in order:
+
+      frames.npy       float64 [n, 4]  stream, logical channel, nbits, offset of the PDU's first byte in frame_bytes
+      frame_bytes.npy  float32 [m]     the packed PDU bytes of those frames, concatenated
+      pids.npy         float32 [n, 12] stream, the 10 PDU bytes, CRC verdict (-1: none)
+      events.npy       float64 [n, 4]  stream, record type (engine.REC_SYNC / REC_LOST_SYNC / REC_MER / REC_BER), then
+                                       frequency offset (Hz), psmi | 0, 0 | lower, upper MER (dB) | channel BER, 0
+      streams.npy      float64 [k]     the streams written
+
+    The sparse event kinds share one array, so that the set of files and their shapes do not depend on whether a
+    workload happens to lose sync; an array that would still be empty is an error, not an empty file.
+
+    When all streams take more than 63 MB, a fixed sample of streams (a permutation seeded with 0, taken while it
+    fits) is written instead, so that two runs with the same arguments write the same streams."""
+    from nrsc5_b200 import engine as eng
+
+    def size(recs):
+        return 8 + sum(4 * len(r["bits"]) + 32 if t == eng.REC_FRAME else 48 for t, r in recs)
+
+    order = np.random.default_rng(0).permutation(len(recs_per_stream))
+    keep, used = [], 0
+    for s in order:
+        used += size(recs_per_stream[s])
+        if used > DUMP_BUDGET_BYTES:
+            break
+        keep.append(int(s))
+    keep.sort()
+    frames, frame_bytes, pids, events = [], [], [], []
+    nbytes = 0
+    for s in keep:
+        for t, r in recs_per_stream[s]:
+            if t == eng.REC_FRAME:
+                frames.append((s, r["lc"], r["nbits"], nbytes))
+                frame_bytes.append(np.frombuffer(r["bits"], dtype=np.uint8))
+                nbytes += len(r["bits"])
+            elif t == eng.REC_PIDS:
+                crc = -1 if r["crc_ok"] is None else r["crc_ok"]
+                pids.append([s, *r["bits"], crc])
+            elif t == eng.REC_SYNC:
+                events.append((s, t, r["freq_offset"], r["psmi"]))
+            elif t == eng.REC_LOST_SYNC:
+                events.append((s, t, 0.0, 0.0))
+            elif t == eng.REC_MER:
+                events.append((s, t, r["lower"], r["upper"]))
+            elif t == eng.REC_BER:
+                events.append((s, t, r["cber"], 0.0))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        "frames": np.array(frames, dtype=np.float64).reshape(-1, 4),
+        "frame_bytes": (np.concatenate(frame_bytes) if frame_bytes else np.zeros(0, np.uint8)).astype(np.float32),
+        "pids": np.array(pids, dtype=np.float32).reshape(-1, 12),
+        "events": np.array(events, dtype=np.float64).reshape(-1, 4),
+        "streams": np.array(keep, dtype=np.float64),
+    }
+    empty = [name for name, a in arrays.items() if a.size == 0]
+    if empty:
+        raise RuntimeError(f"--dump-outputs: the last timed step produced no {', '.join(empty)}")
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -789,6 +860,8 @@ def main():
 
     # ---- value: device-resident ----
     ms, launches, clocks, _ = timed(step_resident, args.steps, max(args.warmup, 3))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, e.drain_all())
     total_samples = samples_per_step * world * args.steps
     value = total_samples / (ms * 1e-3) / 1e6
 

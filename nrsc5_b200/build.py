@@ -5,6 +5,7 @@ library (include/nrsc5_b200.h) that ctypes, cgo or the reference's own C host
 code can bind.
 """
 import os
+import shutil
 import subprocess
 import sys
 
@@ -31,7 +32,9 @@ def _newer(src_paths, out):
 
 
 def build(verbose=False, force=False):
-    nvcc = os.environ.get("NVCC", "nvcc")
+    # nvcc from $NVCC, else PATH, else the toolkit under $CUDA_HOME (a login shell need not put it on PATH)
+    nvcc = (os.environ.get("NVCC") or shutil.which("nvcc")
+            or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc"))
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "nrsc5_b200.h")]
     if not force and not _newer(deps, OUT):
         return OUT

@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (test infrastructure)."""
+import hashlib
 import json
 import lzma
 import os
@@ -8,10 +9,9 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
-SAMPLE_CANDIDATES = [
-    os.path.join(ROOT, "oracle", "_ref", "sample.xz"),   # copied there by build(); travels to the GPU box
-    "/root/reference/support/sample.xz",
-]
+SAMPLE = os.path.join(ROOT, "oracle", "_ref", "sample.xz")    # the reference's support/sample.xz, copied by build()
+# every object of the drop-in libnrsc5.so but the engine (oracle/Makefile)
+DROPIN_OBJDIR = os.path.join(ROOT, "oracle", "_ref", "dropin")
 
 
 def fnv1a32(b: bytes) -> int:
@@ -22,15 +22,39 @@ def fnv1a32(b: bytes) -> int:
 
 
 def load_sample():
-    for p in SAMPLE_CANDIDATES:
-        if os.path.exists(p):
-            return np.frombuffer(lzma.open(p).read(), dtype=np.uint8)
+    if os.path.exists(SAMPLE):
+        return np.frombuffer(lzma.open(SAMPLE).read(), dtype=np.uint8)
     return None
 
 
 def golden(name):
     with open(os.path.join(GOLDEN, name)) as f:
         return json.load(f)
+
+
+REF_DIGESTS = os.path.join(GOLDEN, "reference_digests.json")
+
+
+def digest(value) -> str:
+    """sha256 of repr(value): value is built from ints, Python floats, str, bytes, lists, tuples and dicts."""
+    return hashlib.sha256(repr(value).encode()).hexdigest()
+
+
+def assert_reference(key, got, live=None):
+    """`got` must be what the unmodified reference computes for the same input.  The reference's answer is pinned by
+    its digest in tests/golden/reference_digests.json (made by tests/golden/make_golden_digests.py), so the test
+    needs no reference library; when oracle/_ref holds one, `live()` (the reference's answer, computed now) is checked
+    against that digest as well.  With NRSC5_WRITE_REF_DIGESTS=1 the digest of live() is recorded instead."""
+    import reftap
+    with open(REF_DIGESTS) as f:
+        table = json.load(f)
+    if os.environ.get("NRSC5_WRITE_REF_DIGESTS") == "1":
+        table[key] = digest(live())
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(dict(sorted(table.items())), f, indent=0)
+    elif live is not None and reftap.available():
+        assert digest(live()) == table[key], f"{key}: the reference library disagrees with the committed digest"
+    assert digest(got) == table[key], f"{key}: differs from the unmodified reference"
 
 
 # the synthetic parity matrix (SURVEY §8d): name -> generator kwargs

@@ -2,6 +2,7 @@
 reference's PUBLIC API must deliver the events the unmodified reference delivers - same kinds, same order,
 identical HDC audio packets - on support/sample.xz (golden: tests/golden/api_sample_xz.json, made by
 tests/golden/make_golden_api.py with the unmodified reference)."""
+import json
 import os
 import subprocess
 
@@ -81,18 +82,22 @@ def test_dropin_cs16_pipe_matches_reference_events():
 @pytest.mark.parametrize("psmi,fmt", [(1, "cs16"), (2, "cs16"), (1, "cu8"), (2, "cu8")])
 def test_dropin_am_matches_reference_events(psmi, fmt):
     """AM through the public API (nrsc5_set_mode(NRSC5_MODE_AM), nrsc5_pipe_samples_cs16 / _cu8): the drop-in and
-    the unmodified reference library deliver the same events on a synthetic MA1 / MA3 capture."""
+    the unmodified reference library deliver the same events on a synthetic MA1 / MA3 capture (the reference's events:
+    tests/golden/api_am.json, made by tests/golden/make_golden_api_am.py)."""
     import reftap
     from nrsc5_b200 import synth_am
-    if not os.path.exists(DROPIN) or not reftap.available():
-        pytest.skip("drop-in or reference library not built")
+    if not os.path.exists(DROPIN):
+        pytest.skip("drop-in not built")
     cap = synth_am.make_am_ma1(nframes=8, seed=30 + psmi, lead_in=222, carrier=8000.0, unit=40.0, cfo_hz=0.5, psmi=psmi,
                                flags=(1, 0, 1, 0))
     if fmt == "cs16":
         data, kw = cap.cs16.tobytes(), dict(chunk=32768, cs16=True)
     else:
         data, kw = synth_am.am_to_cu8(cap.cs16).tobytes(), dict(chunk=32768)
-    want = nrsc5_api.run(reftap.REF_SO, data, am=True, **kw)
+    want = common.golden("api_am.json")[f"psmi{psmi}_{fmt}"]
+    if reftap.available():
+        live = json.loads(json.dumps(nrsc5_api.run(reftap.REF_SO, data, am=True, **kw)))
+        assert live == want, "the reference library disagrees with the golden file"
     got = nrsc5_api.run(DROPIN, data, am=True, **kw)
     assert [e[0] for e in want].count("SYNC") == 1 and [e[0] for e in want].count("BER") >= 2
     assert [e[0] for e in got] == [e[0] for e in want]

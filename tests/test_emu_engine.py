@@ -115,7 +115,7 @@ def test_reverse_thread_order_gives_the_same_results():
 def emulated_dropin(emulated_engine):
     import build_emu
     import test_dropin
-    objdir = os.path.join(common.ROOT, "nrsc5_b200", "dropin", "_build", "obj")
+    objdir = common.DROPIN_OBJDIR
     if not os.path.isdir(objdir):
         pytest.skip("drop-in objects not built (needs the reference tree at build time)")
     objs = sorted(os.path.join(objdir, f) for f in os.listdir(objdir) if f.endswith(".o"))

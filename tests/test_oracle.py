@@ -1,6 +1,7 @@
 """CPU tests pinning the oracle (the plain-C restatement in oracle/nrsc5_oracle.c)
 against (1) the committed golden vectors produced by the unmodified reference
-and (2) the reference itself (oracle/_ref/libnrsc5_ref.so) when it is present.
+and (2) the reference's answers on further inputs, pinned by digest (tests/golden/reference_digests.json) and
+recomputed by the reference itself (oracle/_ref/libnrsc5_ref.so) when it is present.
 """
 import ctypes
 
@@ -67,17 +68,19 @@ def test_port_matches_golden_service_modes(name):
         assert len(got) >= least and set(got) <= set(g[key])
 
 
-@pytest.mark.skipif(not reftap.available(), reason="reference oracle not built")
+def _events_and_soft(log):
+    return common.summarize(log), _soft_fnv(log)
+
+
 @pytest.mark.parametrize("psmi", [2, 5, 11])
 def test_port_matches_reference_live_service_modes(psmi):
     """The restatement against the unmodified reference on a capture that is not in the golden file (other seed,
     start block and noise), so that the pin does not rest on four inputs only."""
     cap = synth.make_fm(psmi=psmi, nframes=3, seed=100 + psmi, lead_in=1234, tail_blocks=2, cfo_hz=-150.0, noise_lsb=10.0,
                         start_bc=5)
-    ref = reftap.decode(cap.cu8, want_soft=True)
     log = port.decode(cap.cu8, want_soft=True)
-    assert common.summarize(log) == common.summarize(ref)
-    assert _soft_fnv(log) == _soft_fnv(ref)
+    common.assert_reference(f"fm_service_mode_psmi{psmi}", _events_and_soft(log),
+                            lambda: _events_and_soft(reftap.decode(cap.cu8, want_soft=True)))
 
 
 def test_port_matches_golden_sample():
@@ -95,15 +98,12 @@ def test_port_matches_golden_sample():
     assert kinds.count("B") == 9 and kinds.count("F") == 9 and kinds.count("P") == 172
 
 
-@pytest.mark.skipif(not reftap.available(), reason="reference oracle not built")
 def test_port_cs16_matches_reference():
     """input_push_cs16: the reference and the restatement on the same pre-decimated FM capture."""
     cap = synth.make_fm_mp1(nframes=1, seed=21, lead_in=64, cfo_hz=50.0)
     cs16 = port.halfband_fm(cap.cu8[: cap.cu8.size & ~3])
     a = port.decode(cs16, want_soft=True)
-    b = reftap.decode(cs16, want_soft=True)
-    assert common.summarize(a) == common.summarize(b)
-    assert _soft_fnv(a) == _soft_fnv(b)
+    common.assert_reference("fm_cs16", _events_and_soft(a), lambda: _events_and_soft(reftap.decode(cs16, want_soft=True)))
     # and the decimator in front of it changes nothing: the cu8 capture gives the same PDUs
     c = port.decode(cap.cu8)
     assert [e for e in common.summarize(c) if e[0] in "FP"] == [e for e in common.summarize(a) if e[0] in "FP"]
@@ -117,72 +117,100 @@ def test_port_chunking_invariance():
     assert common.summarize(a) == common.summarize(b) == common.summarize(c)
 
 
-@pytest.mark.skipif(not reftap.available(), reason="reference oracle not built")
+def _records(log):
+    """A decode's records, the reference tap's HDC records and the oracle's own PIDS CRC verdict left out, numpy
+    arrays as bytes."""
+    return [(t, {k: (v.tobytes() if isinstance(v, np.ndarray) else v) for k, v in r.items() if k != "crc_ok"})
+            for t, r in log.records if t != reftap.REC_HDC]
+
+
+def _ptr(a):
+    return a.ctypes.data_as(ctypes.c_void_p)
+
+
 class TestAgainstReference:
     def test_full_chain_noisy(self):
         cap = synth.make_fm_mp1(nframes=1, seed=21, lead_in=123, cfo_hz=-150.0, noise_lsb=10.0)
-        a = reftap.decode(cap.cu8, want_soft=True)
         b = port.decode(cap.cu8, want_soft=True)
-        ra = [r for r in a.records if r[0] != reftap.REC_HDC]
-        assert len(ra) == len(b.records)
-        for x, y in zip(ra, b.records):
-            assert x[0] == y[0]
-            if x[0] == reftap.REC_SOFT_PM:
-                assert x[1]["bc"] == y[1]["bc"] and np.array_equal(x[1]["soft"], y[1]["soft"])
-            else:
-                # (the CRC verdict of a PIDS record is the oracle's own addition, the reference tap has none)
-                assert {k: v for k, v in x[1].items() if k != "crc_ok"} == {k: v for k, v in y[1].items() if k != "crc_ok"}
+        common.assert_reference("fm_full_chain_noisy", _records(b), lambda: _records(reftap.decode(cap.cu8, want_soft=True)))
 
     def test_viterbi_k7_k9(self):
-        L = reftap.lib()
         rng = np.random.default_rng(1)
-        for n in (80, 2304, 4608):
-            soft = rng.integers(-127, 128, 3 * n, dtype=np.int8)
-            out = np.empty(n, dtype=np.uint8)
-            L.nrsc5_conv_decode_p3_p4(soft.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p), n)
-            assert np.array_equal(out, port.viterbi(soft))
-        soft = rng.integers(-1, 2, 3 * 3750, dtype=np.int8)
-        out = np.empty(3750, dtype=np.uint8)
-        L.nrsc5_conv_decode_e1(soft.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p), 3750)
-        assert np.array_equal(out, port.viterbi(soft, k=9, gens=(0o561, 0o657, 0o711)))
-        L.nrsc5_conv_decode_e2_e3(soft.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p), 3750)
-        assert np.array_equal(out, port.viterbi(soft, k=9, gens=(0o561, 0o753, 0o711)))
+        soft7 = [rng.integers(-127, 128, 3 * n, dtype=np.int8) for n in (80, 2304, 4608)]
+        soft9 = rng.integers(-1, 2, 3 * 3750, dtype=np.int8)
+        e1, e23 = (0o561, 0o657, 0o711), (0o561, 0o753, 0o711)
+        got = [port.viterbi(s).tobytes() for s in soft7]
+        got += [port.viterbi(soft9, k=9, gens=e1).tobytes(), port.viterbi(soft9, k=9, gens=e23).tobytes()]
+
+        def live():
+            L = reftap.lib()
+            outs = []
+            for s in soft7:
+                out = np.empty(s.size // 3, dtype=np.uint8)
+                L.nrsc5_conv_decode_p3_p4(_ptr(s), _ptr(out), out.size)
+                outs.append(out.tobytes())
+            for f in (L.nrsc5_conv_decode_e1, L.nrsc5_conv_decode_e2_e3):
+                out = np.empty(3750, dtype=np.uint8)
+                f(_ptr(soft9), _ptr(out), 3750)
+                outs.append(out.tobytes())
+            return outs
+        common.assert_reference("viterbi_k7_k9", got, live)
 
     def test_viterbi_saturation(self):
         # full-scale, perfectly consistent, unpunctured input drives the int16
         # path metrics into saturation between normalisations (SURVEY §7.3)
-        L = reftap.lib()
         rng = np.random.default_rng(5)
         u = rng.integers(0, 2, 4608, dtype=np.uint8)
         c = synth.conv_encode_tb(u).reshape(-1).astype(np.int16)
         s = ((2 * c - 1) * 127).astype(np.int8)
-        out = np.empty(4608, dtype=np.uint8)
-        L.nrsc5_conv_decode_p3_p4(s.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p), 4608)
-        assert np.array_equal(out, port.viterbi(s)) and np.array_equal(out, u)
+        got = port.viterbi(s)
+        assert np.array_equal(got, u)
+
+        def live():
+            out = np.empty(4608, dtype=np.uint8)
+            reftap.lib().nrsc5_conv_decode_p3_p4(_ptr(s), _ptr(out), 4608)
+            return out.tobytes()
+        common.assert_reference("viterbi_saturation", got.tobytes(), live)
 
     def test_halfband(self):
-        L = reftap.lib()
-        L.firdecim_q15_create.restype = ctypes.c_void_p
-        L.halfband_q15_execute.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
-        taps = (ctypes.c_float * 4)(0.6062333583831787, -0.13481467962265015, 0.032919470220804214, -0.00410953676328063)
-        q = L.firdecim_q15_create(taps, 4)
         rng = np.random.default_rng(2)
         cu8 = rng.integers(0, 256, 4 * 5000, dtype=np.uint8)
         cu8[:400] = 255                      # extremes
         cu8[400:800] = 0
-        x = ((cu8.astype(np.int16) - 127) * 64).astype(np.int16)
-        out = np.empty(2 * 5000, dtype=np.int16)
-        for n in range(5000):
-            L.halfband_q15_execute(q, x[4 * n:].ctypes.data_as(ctypes.c_void_p),
-                                   out[2 * n:].ctypes.data_as(ctypes.c_void_p))
-        assert np.array_equal(out, port.halfband_fm(cu8))
 
-    def test_rs_decode(self):
+        def live():
+            L = reftap.lib()
+            L.firdecim_q15_create.restype = ctypes.c_void_p
+            L.halfband_q15_execute.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+            taps = (ctypes.c_float * 4)(0.6062333583831787, -0.13481467962265015, 0.032919470220804214, -0.00410953676328063)
+            q = L.firdecim_q15_create(taps, 4)
+            x = ((cu8.astype(np.int16) - 127) * 64).astype(np.int16)
+            out = np.empty(2 * 5000, dtype=np.int16)
+            for n in range(5000):
+                L.halfband_q15_execute(q, _ptr(x[4 * n:]), _ptr(out[2 * n:]))
+            return out.tobytes()
+        common.assert_reference("halfband", port.halfband_fm(cu8).tobytes(), live)
+
+    @staticmethod
+    def _ref_rs(blocks):
         L = reftap.lib()
         L.init_rs_char.restype = ctypes.c_void_p
         L.decode_rs_char.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
         rs = L.init_rs_char(8, 0x11D, 1, 1, 8)
+        out = []
+        for blk in blocks:
+            ref = blk.copy()
+            rc = L.decode_rs_char(rs, _ptr(ref), None, 0)
+            out.append((rc, ref.tobytes()))
+        return out
+
+    @staticmethod
+    def _port_rs(blocks):
+        return [(rc, got.tobytes()) for rc, got in (port.rs_decode(blk) for blk in blocks)]
+
+    def test_rs_decode(self):
         rng = np.random.default_rng(7)
+        blocks = []
         for t in range(1500):
             hdr = np.frombuffer(synth.audio_pdu_header(rng=rng), dtype=np.uint8)
             blk = np.zeros(255, dtype=np.uint8)
@@ -191,28 +219,17 @@ class TestAgainstReference:
                 blk[p if t % 3 == 0 else 254 - p] ^= rng.integers(1, 256)
             if t % 50 == 49:
                 blk = rng.integers(0, 256, 255, dtype=np.uint8)
-            ref = blk.copy()
-            rc_ref = L.decode_rs_char(rs, ref.ctypes.data_as(ctypes.c_void_p), None, 0)
-            rc, got = port.rs_decode(blk)
-            assert rc == rc_ref and np.array_equal(ref, got)
+            blocks.append(blk)
+        common.assert_reference("rs_decode", self._port_rs(blocks), lambda: self._ref_rs(blocks))
 
     def test_rs_decode_beyond_the_radius(self):
         """The words of tests/test_gpu_stages.py::test_rs_beyond_the_correction_radius_equals_reference (5..8 symbol
         errors): the oracle's decoder = the unmodified reference's decode_rs_char, including every mis-correction."""
         import test_gpu_stages
-        L = reftap.lib()
-        L.init_rs_char.restype = ctypes.c_void_p
-        L.decode_rs_char.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
-        rs = L.init_rs_char(8, 0x11D, 1, 1, 8)
         blocks = test_gpu_stages._rs_words(np.random.default_rng(2024), 120000)
-        ncorr = 0
-        for blk in blocks:
-            ref = blk.copy()
-            rc_ref = L.decode_rs_char(rs, ref.ctypes.data_as(ctypes.c_void_p), None, 0)
-            rc, got = port.rs_decode(blk)
-            assert rc == rc_ref and np.array_equal(ref, got)
-            ncorr += rc_ref > 0
-        assert ncorr > 50
+        got = self._port_rs(blocks)
+        common.assert_reference("rs_decode_beyond_the_radius", got, lambda: self._ref_rs(blocks))
+        assert sum(rc > 0 for rc, _ in got) > 50
 
 
 def test_rs_roundtrip_without_reference():

@@ -1,5 +1,6 @@
 """CPU tests pinning the AM restatement (oracle/nrsc5_oracle_am.c) against the UNMODIFIED reference
-(oracle/_ref/libnrsc5_ref.so, AM mode) and the committed golden file, on the synthetic MA1 and MA3 captures."""
+(oracle/_ref/libnrsc5_ref.so, AM mode; pinned by digest in tests/golden/reference_digests.json) and the committed
+golden file, on the synthetic MA1 and MA3 captures."""
 import pytest
 
 import common
@@ -22,13 +23,12 @@ def test_am_port_matches_golden(name):
     assert kinds.count("S") == 1 and kinds.count("B") >= 4 and kinds.count("P") >= 60
 
 
-@pytest.mark.skipif(not reftap.available(), reason="reference oracle not built")
 @pytest.mark.parametrize("psmi", [1, 2])
 def test_am_port_matches_reference_and_is_chunking_invariant(psmi):
     cap = synth_am.make_am_ma1(nframes=9, seed=9, lead_in=1234, cfo_hz=-0.8, noise_lsb=5.0, psmi=psmi)
-    ref = reftap.decode(cap.cs16, mode=reftap.MODE_AM)
     a = port.decode_am(cap.cs16)
     b = port.decode_am(cap.cs16, chunk=16384)
     c = port.decode_am(cap.cs16, chunk=2 * 977)
-    assert common.summarize(a) == common.summarize(ref)
+    common.assert_reference(f"am_psmi{psmi}", common.summarize(a),
+                            lambda: common.summarize(reftap.decode(cap.cs16, mode=reftap.MODE_AM)))
     assert common.summarize(a) == common.summarize(b) == common.summarize(c)

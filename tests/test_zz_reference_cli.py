@@ -5,7 +5,7 @@
     support/cli.py -r sample -o sample.wav 0      ; same grep
 
 with `nrsc5` = the reference's UNMODIFIED command-line program (src/main.c + src/log.c, compiled where they lie by
-tests/cli/build_cli.py, libao replaced by a byte-counting stand-in) linked against the drop-in libnrsc5.so, and
+oracle/Makefile, linked by tests/cli/build_cli.py, libao replaced by a byte-counting stand-in) against the drop-in libnrsc5.so, and
 `support/cli.py` = the reference's unmodified Python CLI loading the drop-in through its own ctypes binding
 (support/nrsc5.py:676-690).  This is the claim of BASELINE.json's north_star - "the CLI and Python bindings drop in
 unchanged" - tested the way the reference tests itself.  Beyond the grep, every information line the CLI prints
@@ -13,7 +13,7 @@ unchanged" - tested the way the reference tests itself.  Beyond the grep, every 
 against the unmodified reference library.
 
 CPU tier: the drop-in on the CPU emulation of the kernels (tests/emu), first 20 MB of the capture.
-GPU tier: the real drop-in, whole capture; the binaries are built by __graft_entry__.build() and travel to the box.
+GPU tier: the real drop-in, whole capture; the binaries are linked by __graft_entry__.build() from oracle/_ref/.
 """
 import os
 import re
@@ -31,7 +31,7 @@ import build_cli  # noqa: E402
 
 BUILD = os.path.join(HERE, "_build")
 GREP = "You're Listening to Q"
-REF_SUPPORT = "/root/reference/support"
+REF_SUPPORT = os.path.join(common.ROOT, "oracle", "_ref", "support")   # the reference's support/*.py, copied by build()
 
 
 def info_lines(log: str):
@@ -80,7 +80,7 @@ def control_binary():
 def emulated_cli():
     """libnrsc5.so = the drop-in's objects on the emulated engine, and the reference CLI linked against it."""
     import build_emu
-    objdir = os.path.join(common.ROOT, "nrsc5_b200", "dropin", "_build", "obj")
+    objdir = common.DROPIN_OBJDIR
     if not build_cli.available() or not os.path.isdir(objdir):
         pytest.skip("needs the reference tree (the CLI and the drop-in's host objects are compiled from it)")
     emu = build_emu.build()
